@@ -2,7 +2,7 @@
 """bench.py — images/sec of feather::Net::Forward on synthetic 224x224x3 input (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--model vgg16|resnet50|mobilenet_v1|single_conv]
-                    [--batch B_per_gpu] [--precision tf32x3|tf32] [--impl b200|reference]
+                    [--batch B_per_gpu] [--precision tf32x3|tf32] [--impl b200|reference] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...      (one rank per GPU, NCCL)
 
 One "step" = one Forward over one batch.  Default workload = BASELINE.json configs[1]: VGG-16 fp32, batch 64 per
@@ -17,6 +17,8 @@ Prints ONE JSON line on rank 0:
                 MEASURED_PEAKS.json) and lists the others under other_kernels
   cpu_baseline  the unmodified reference (oracle/_ref) on the host cores, bounded sample, rank 0 / N=1 only
 `--impl reference` times only that CPU reference arm (no GPU work) and prints the same line shape.
+`--dump-outputs DIR` writes, on rank 0, the output blob of the last timed step of each workload as DIR/<model>_<blob>.npy
+(float32, batch x C x H x W); the inputs and weights are seeded, so two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -36,6 +38,7 @@ sys.path.insert(0, str(ROOT))
 
 DEFAULT_BATCH = {"vgg16": 64, "resnet50": 128, "mobilenet_v1": 256, "single_conv": 64}
 L2_BYTES = 126 * 1024 * 1024
+DUMP_BYTES_PER_WORKLOAD = 16 << 20  # at most three workloads: 48 MB in all
 
 
 def env_int(name: str, default: int) -> int:
@@ -309,6 +312,27 @@ def parity_gate(net, param: str, binf: str, in_shape, batch: int, image_index: i
         return {"parity_max_rel": None, "pass": False, "error": f"{type(e).__name__}: {e}"[:300]}
 
 
+def rotating_batches(batch_bytes: int) -> int:
+    """How many input batches the timed steps rotate through: together larger than L2, at least 2, at most 8."""
+    return min(8, max(2, -(-int(1.25 * L2_BYTES) // batch_bytes)))
+
+
+def input_batch(in_shape, B: int, rank: int, n_rot: int, r: int) -> np.ndarray:
+    """Rotating batch r of `rank`: four seeded synthetic images repeated to B; step i feeds batch i % n_rot."""
+    from feathercnn_b200.tools import modelgen
+    base = np.stack([modelgen.synthetic_input(in_shape, (rank * n_rot + r) * 4 + i) for i in range(min(B, 4))])
+    return np.resize(base, (B,) + tuple(in_shape))
+
+
+def dump_output(net, out_name: str, model: str, out_dir: Path) -> None:
+    """What the last timed Forward left in the output blob, as a caller would Extract it; past the per-workload byte
+    budget only the first images are kept (a fixed sample)."""
+    out = np.ascontiguousarray(net.Extract(out_name), np.float32)
+    keep = max(1, DUMP_BYTES_PER_WORKLOAD // max(1, out[0].nbytes))
+    out_dir.mkdir(parents=True, exist_ok=True)
+    np.save(out_dir / f"{model}_{out_name}.npy", out[:keep])
+
+
 def run_workload(args, model: str, B: int, rank: int, world: int, local_rank: int, barrier, full: bool,
                  cpu_leg: bool) -> dict | None:
     """Loads `model`, times the device-resident and end-to-end legs on every rank; rank 0 returns the result dict."""
@@ -328,16 +352,14 @@ def run_workload(args, model: str, B: int, rank: int, world: int, local_rank: in
     t_load = time.perf_counter() - t_load
 
     batch_bytes = B * int(np.prod(in_shape)) * 4
-    n_rot = max(2, -(-int(1.25 * L2_BYTES) // batch_bytes))  # rotating inputs larger than L2 in total
-    n_rot = min(n_rot, 8)
+    n_rot = rotating_batches(batch_bytes)
     host_batches = []
     for r in range(n_rot):
         hb = torch.empty((B,) + tuple(in_shape), dtype=torch.float32).pin_memory()
-        base = np.stack([modelgen.synthetic_input(in_shape, (rank * n_rot + r) * 4 + i) for i in range(min(B, 4))])
-        hb.copy_(torch.from_numpy(np.resize(base, (B,) + tuple(in_shape))))
+        hb.copy_(torch.from_numpy(input_batch(in_shape, B, rank, n_rot, r)))
         host_batches.append(hb)
     dev_batches = [hb.to(dev) for hb in host_batches]
-    out_name = "prob" if "prob" in net.BlobNames() else sorted(net.BlobNames())[-1]
+    out_name = "prob" if "prob" in net.BlobNames() else sorted(b for b in net.BlobNames() if b != "data")[-1]
     torch.cuda.synchronize(dev)
 
     def max_over_ranks(ms: float) -> float:
@@ -376,6 +398,8 @@ def run_workload(args, model: str, B: int, rank: int, world: int, local_rank: in
         if sampler:
             sampler.end()
         ms_dev = max_over_ranks(e0.elapsed_time(e1))
+        if args.dump_outputs and rank == 0:
+            dump_output(net, out_name, model, Path(args.dump_outputs))
 
         if args.lean:
             if sampler:
@@ -494,7 +518,11 @@ def main() -> None:
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--l2-chunk-mb", type=float, default=None)
     ap.add_argument("--lean", action="store_true", help="profiling aid: device-resident leg only (no e2e / roofline / cpu legs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the output blob of the last timed step of each workload to DIR/<model>_<blob>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     headline = args.model or "vgg16"
     extra = [] if (args.model or args.lean) else ["resnet50", "mobilenet_v1"]
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup

@@ -23,6 +23,40 @@ def rel_err(got: np.ndarray, ref: np.ndarray) -> float:
     return float(np.abs(got - ref).max()) / denom
 
 
+def sample_index(size: int, n: int = 512) -> np.ndarray:
+    """n flat indices spread over an array of `size` elements (a fixed stride modulo a prime), or all of them."""
+    if size <= n:
+        return np.arange(size)
+    return np.arange(n, dtype=np.int64) * 1000003 % size
+
+
+def sample_of(ref: np.ndarray) -> dict:
+    """What tests/golden/ keeps of a large reference output: its values at sample_index and max|ref| over the whole
+    array (the denominator of rel_err)."""
+    ref = np.asarray(ref, np.float32).reshape(-1)
+    return {"val": ref[sample_index(ref.size)], "amax": np.float32(np.abs(ref).max())}
+
+
+def sampled_rel_err(got: np.ndarray, gold, key: str) -> float:
+    """rel_err against a stored sample (sample_of, saved under `key`/val and `key`/amax): max|got - ref| over the
+    sampled elements / max|ref| over the whole reference array."""
+    got = np.asarray(got, np.float64).reshape(-1)
+    want = gold[key + "/val"]
+    got = got[sample_index(got.size)]
+    assert got.shape == want.shape, (got.shape, want.shape)
+    return float(np.abs(got - want).max()) / max(float(gold[key + "/amax"]), 1e-30)
+
+
+def digest(*arrays) -> str:
+    """sha256 of the arrays' bytes: pins the regenerated inputs of a golden comparison to the ones it was made from."""
+    import hashlib
+    h = hashlib.sha256()
+    for a in arrays:
+        if a is not None:
+            h.update(np.ascontiguousarray(a).tobytes())
+    return h.hexdigest()
+
+
 @pytest.fixture(scope="session")
 def oracle():
     from oracle import oracle as O
@@ -33,13 +67,6 @@ def oracle():
 @pytest.fixture(scope="session")
 def restatement(oracle):
     return oracle.restatement()
-
-
-@pytest.fixture(scope="session")
-def reference(oracle):
-    if not oracle.reference_available():
-        pytest.skip("oracle/_ref/libfeather_ref.so not built (needs /root/reference at build time)")
-    return oracle.Reference()
 
 
 @pytest.fixture(scope="session")

@@ -1,13 +1,14 @@
 """GPU parity of the convolution hot path (SURVEY.md §8 rows a1-a11) through the C ABI (include/fcuda.h),
-against the oracle restatement (oracle/feather_oracle.c) and, when present, the unmodified reference build
-(oracle/_ref).  Tolerances: 3xTF32 (default, fp32-equivalent) 2e-4 of max|ref| per layer — the reference's own
+against the oracle restatement (oracle/feather_oracle.c) and outputs of the unmodified reference build stored under
+tests/golden/.  Tolerances: 3xTF32 (default, fp32-equivalent) 2e-4 of max|ref| per layer — the reference's own
 Winograd path is ~1e-5 from an fp64 convolution; plain TF32 is held to the north-star bar of 1e-3."""
 import ctypes
+from pathlib import Path
 
 import numpy as np
 import pytest
 
-from conftest import rel_err
+from conftest import digest, rel_err, sampled_rel_err
 
 pytestmark = pytest.mark.gpu
 
@@ -90,13 +91,15 @@ REF_CASES = [c for c in CASES[:14] if c[0] != "wino_min_size"]
 
 
 @pytest.mark.parametrize("case", REF_CASES, ids=[c[0] for c in REF_CASES])
-def test_conv_matches_reference_build(cuda, oracle, reference, case):
+def test_conv_matches_reference_build(cuda, oracle, case):
+    """Against a fixed sample of the reference's ConvBooster output (tests/golden/make_golden.py)."""
     from feathercnn_b200 import booster
     booster.set_precision(booster.PRECISION_TF32X3)
+    gold = np.load(Path(__file__).resolve().parent / "golden" / "ref_gpu_conv.npz")
     p, x, wt, b = _data(oracle, case, 1, seed=7)
+    assert digest(x, wt, b) == str(gold[case[0] + "/inputs"]), "inputs differ from those the stored outputs were made from"
     got, _ = _gpu_conv(cuda, case, x, wt, b)
-    want = reference.conv(p, x[0], wt, b)
-    assert rel_err(got[0], want) < 2e-4, case[0]
+    assert sampled_rel_err(got[0], gold, case[0]) < 2e-4, case[0]
 
 
 @pytest.mark.parametrize("algo_name", ["NAIVE", "IM2COL", "SGECONV", "WINOGRADF63", "WINOGRADF23"])

@@ -304,3 +304,37 @@ def test_net_group_one_process_many_devices(cuda, model_dir, ndev):
             assert g.Member(i).BlobShape("prob")[0] == hi - lo
         del g
     cuda.cuda.set_device(0)
+
+
+def test_bench_dump_outputs_is_the_last_timed_step(cuda, oracle, tmp_path):
+    """bench.py --dump-outputs: the output blob of the last timed step — the oracle's Forward of the batch that step fed
+    (bench.input_batch) — and the same from run to run (seeded inputs and weights), so two builds can be compared
+    output for output."""
+    import importlib.util
+    import os
+    import subprocess
+    import sys
+    from pathlib import Path
+    root = Path(__file__).resolve().parent.parent
+    spec = importlib.util.spec_from_file_location("bench_mod", root / "bench.py")
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    cache = tmp_path / "models"
+    env = dict(os.environ, FEATHER_BENCH_CACHE=str(cache))
+    batch, steps, in_shape = 4, 3, (64, 56, 56)
+    outs = []
+    for run in ("a", "b"):
+        cmd = [sys.executable, str(root / "bench.py"), "--model", "single_conv", "--batch", str(batch), "--steps", str(steps),
+               "--warmup", "0", "--lean", "--dump-outputs", str(tmp_path / run)]
+        r = subprocess.run(cmd, capture_output=True, text=True, timeout=600, cwd=root, env=env)
+        assert r.returncode == 0, r.stderr[-2000:]
+        assert [f.name for f in (tmp_path / run).iterdir()] == ["single_conv_conv.npy"]
+        outs.append(np.load(tmp_path / run / "single_conv_conv.npy"))
+    assert outs[0].dtype == np.float32 and outs[0].shape == (batch, 64, 56, 56)
+    np.testing.assert_array_equal(outs[0], outs[1])
+    n_rot = bench.rotating_batches(batch * int(np.prod(in_shape)) * 4)
+    x = bench.input_batch(in_shape, batch, 0, n_rot, (steps - 1) % n_rot)
+    cpu = oracle.OracleNet(cache / "single_conv_seed0.param", cache / "single_conv_seed0.bin")
+    for n in range(batch):
+        cpu.forward(x[n])
+        assert rel_err(outs[0][n], cpu.extract("conv")) < 2e-4, n

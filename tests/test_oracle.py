@@ -2,8 +2,9 @@
 
 1. the C restatement (oracle/feather_oracle.c) and the NumPy net interpreter reproduce the committed golden
    fixtures, which are outputs of the UNMODIFIED reference (tests/golden/make_golden.py);
-2. when oracle/_ref is built (authoring container, GPU box via the travelling .so) the restatement also agrees
-   with the live reference over the shape sweep used by the GPU tests;
+2. the restatement also agrees with the reference's outputs over the shape sweep used by the GPU tests, the
+   reference's Forward of a second net, and its pixel staging (stored from the unmodified reference by
+   tests/golden/make_golden.py: fixed samples of the float outputs, digests of the bit-exact ones);
 3. both agree with an independent fp64 direct convolution, so an oracle bug cannot silently become the spec.
 """
 from pathlib import Path
@@ -11,7 +12,7 @@ from pathlib import Path
 import numpy as np
 import pytest
 
-from conftest import rel_err
+from conftest import digest, rel_err, sampled_rel_err
 
 GOLD = Path(__file__).resolve().parent / "golden"
 
@@ -77,35 +78,51 @@ SWEEP = [
 ]
 
 
-@pytest.mark.parametrize("geom", SWEEP)
-def test_restatement_vs_live_reference_and_fp64(oracle, restatement, reference, geom):
+def sweep_data(oracle, geom):
     p = _param(oracle, geom)
     rng = np.random.default_rng(11)
     x = rng.uniform(-0.5, 0.5, (p.input_channels, p.input_h, p.input_w)).astype(np.float32)
     w = (rng.standard_normal(p.weight_shape) * 0.05).astype(np.float32)
     b = rng.uniform(-0.1, 0.1, p.output_channels).astype(np.float32) if p.bias_term else None
-    want = reference.conv(p, x, w, b)
+    return p, x, w, b
+
+
+@pytest.mark.parametrize("geom", SWEEP)
+def test_restatement_vs_live_reference_and_fp64(oracle, restatement, geom):
+    """The restatement against the reference's ConvBooster output on the sweep, read from tests/golden/ref_conv_sweep.npz
+    (a fixed sample of each output, stored by make_golden.py), and against the fp64 direct convolution in full; the
+    reference's own NAIVE path, stored the same way, against fp64."""
+    gold = np.load(GOLD / "ref_conv_sweep.npz")
+    key = str(SWEEP.index(geom))
+    p, x, w, b = sweep_data(oracle, geom)
+    assert digest(x, w, b) == str(gold[key + "/inputs"]), "inputs differ from those the stored outputs were made from"
     got = restatement.conv(p, x, w, b)
-    assert rel_err(got, want) < 5e-5
+    assert sampled_rel_err(got, gold, key + "/ref") < 5e-5
     if p.group == 1:
         f64 = restatement.conv(p, x, w, b, f64=True)
-        assert rel_err(want, f64) < 5e-5 and rel_err(got, f64) < 5e-5
-        naive = reference.conv(p, x, w, b, algo=oracle.ALGO_NAIVE)  # the authors' own oracle, avx/booster.cpp:28-61
-        if not p.activation:  # NAIVE_Forward ignores the activation field
-            assert rel_err(naive, f64) < 5e-6
+        assert sampled_rel_err(f64, gold, key + "/ref") < 5e-5 and rel_err(got, f64) < 5e-5
+        if not p.activation:  # the authors' own oracle, avx/booster.cpp:28-61; NAIVE_Forward ignores the activation field
+            assert sampled_rel_err(f64, gold, key + "/naive") < 5e-6
 
 
-def test_net_interpreter_vs_live_reference_net(oracle, reference, tmp_path):
+def mini3(tmp_path):
+    """modelgen.mini(seed=3) and its synthetic image 5: the second net the interpreter is checked on."""
     from feathercnn_b200.tools import modelgen
     m = modelgen.mini(seed=3)
     param, binf = m.save(tmp_path / "mini")
-    x = modelgen.synthetic_input(m.shape["data"], 5)
-    rn = oracle.ReferenceNet(param, binf)
-    rn.forward(x)
+    return m, param, binf, modelgen.synthetic_input(m.shape["data"], 5)
+
+
+def test_net_interpreter_vs_live_reference_net(oracle, tmp_path):
+    """Every blob of the interpreter's Forward of modelgen.mini(seed=3) against the reference's feather::Net::Forward,
+    read from tests/golden/ref_mini_seed3.npz (a fixed sample of each blob, stored by make_golden.py)."""
+    gold = np.load(GOLD / "ref_mini_seed3.npz")
+    m, param, binf, x = mini3(tmp_path)
+    assert digest(x, np.frombuffer(Path(param).read_bytes(), np.uint8), np.fromfile(binf, np.uint8)) == str(gold["inputs"])
     on = oracle.OracleNet(param, binf)
     on.forward(x)
     for b in sorted(m.blobs):
-        assert rel_err(on.extract(b), rn.extract(b)) < 5e-5, b
+        assert sampled_rel_err(on.extract(b), gold, b) < 5e-5, b
 
 
 def test_pooling_quirks(restatement):
@@ -123,17 +140,30 @@ PIXEL_TYPES = [(1, 3), (2, 3), (4, 1), (8, 4), (1 | (2 << 16), 3), (2 | (1 << 16
                (4 | (1 << 16), 1), (4 | (2 << 16), 1), (8 | (1 << 16), 4), (8 | (2 << 16), 4), (8 | (4 << 16), 4)]
 
 
-def test_pixel_staging_restatement_is_bit_exact_with_the_reference(oracle, reference):
+PIXEL_SIZES = [(32, 48, 24, 24), (37, 53, 224, 224), (64, 64, 64, 64), (240, 320, 224, 224), (17, 9, 40, 31), (2, 2, 5, 7)]
+
+
+def pixel_cases():
+    """(h, w, tw, th, type, image) in the order the stored reference digests were made."""
+    rng = np.random.default_rng(0)
+    for (h, w, tw, th) in PIXEL_SIZES:
+        for t, c in PIXEL_TYPES:
+            yield h, w, tw, th, t, rng.integers(0, 256, (h, w, c), dtype=np.uint8)
+
+
+def test_pixel_staging_restatement_is_bit_exact_with_the_reference(oracle):
     """Input staging (SURVEY.md §8f rank 3): the NumPy restatement of ncnn::Mat::from_pixels / from_pixels_resize
     (mat_pixel.cpp:1329-1410, mat_pixel_resize.cpp:26-278 — u8 fixed-point bilinear, byte work: bit-exact bar) against the
     unmodified reference, every pixel type, up- and down-scaling, degenerate 2x2 sources."""
-    rng = np.random.default_rng(0)
-    for (h, w, tw, th) in [(32, 48, 24, 24), (37, 53, 224, 224), (64, 64, 64, 64), (240, 320, 224, 224), (17, 9, 40, 31), (2, 2, 5, 7)]:
-        for t, c in PIXEL_TYPES:
-            img = rng.integers(0, 256, (h, w, c), dtype=np.uint8)
-            want = reference.from_pixels(img, t, tw, th)
-            got = oracle.from_pixels(img, t, tw, th)
-            assert want is not None and got is not None and got.shape == want.shape
-            np.testing.assert_array_equal(got, want, err_msg=f"type {t:#x} {w}x{h}->{tw}x{th}")
+    import json
+    gold = json.loads((GOLD / "ref_from_pixels.json").read_text())
+    cases = list(pixel_cases())
+    assert len(cases) == len(gold["cases"]) == len(PIXEL_SIZES) * len(PIXEL_TYPES)
+    for (h, w, tw, th, t, img), want in zip(cases, gold["cases"]):
+        what = f"type {t:#x} {w}x{h}->{tw}x{th}"
+        assert digest(img) == want["image"], what + ": input differs from the one the stored output was made from"
+        got = oracle.from_pixels(img, t, tw, th)
+        assert got is not None and list(got.shape) == want["shape"], what
+        assert digest(got) == want["output"], what
     assert oracle.from_pixels(np.zeros((4, 4, 3), np.uint8), 3) is None          # unknown type: empty Mat upstream
-    assert reference.from_pixels(np.zeros((4, 4, 3), np.uint8), 3) is None
+    assert gold["unknown_type"] is None
